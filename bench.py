@@ -2,6 +2,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this package (CUDA kernels through the C ABI)
   python bench.py --impl reference --gpus N --steps K ...   # the reference path's CPU port (oracle) on the host cores
+  python bench.py ... --dump-outputs DIR                    # also write the last timed step's latents to DIR/*.npy
 
 Workload (BASELINE.json configs[1], the configuration the metric is quoted on): one 16-frame 512x512 clip
 (latents [1,4,16,64,64]), full-size random-init I2VGen-XL UNet (1.42 B params, fp16), 50-step schedules, guidance 9.0,
@@ -211,6 +212,13 @@ def run_ours(args):
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    # what the last timed step of each phase returned to its caller, copied before the passes below reuse the static buffers
+    last_outputs = {}
+    if args.dump_outputs:
+        if k_inv:
+            last_outputs["inversion_latents"] = st_inv.latents.float().cpu()
+        if k_edit:
+            last_outputs["edit_latents"] = st_edit.latents.float().cpu()
     graphs = pipe.use_cuda_graphs
     # kernels launched per replayed step are the ones recorded at capture time
     launches = ops.launch_count() - l0
@@ -301,7 +309,25 @@ def run_ours(args):
         out["metric"] = METRIC.replace("16f", f"{F}f")
     if not args.no_cpu_baseline and world >= 1:
         out["cpu_baseline"] = cpu_baseline(budget_s=args.cpu_budget)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_outputs)
     print(json.dumps(out), flush=True)
+
+
+DUMP_BYTES = 60 * 2 ** 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy in float32, DUMP_BYTES at most in all.  An array larger than its share is replaced by
+    a seeded sample of its elements, the same positions in every run, so that two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // 4 // max(len(arrays), 1)
+    for name, t in arrays.items():
+        if t.numel() > share:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:share].sort().values
+            t = t.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.numpy().astype(np.float32))
 
 
 def attention_roofline(ops, dev):
@@ -684,7 +710,14 @@ def main():
     ap.add_argument("--frames", type=int, default=16, help="frames per clip: 16 (BASELINE configs[1], default) or 128 (configs[4])")
     ap.add_argument("--cpu-budget", type=float, default=40.0)
     ap.add_argument("--ref-budget", type=float, default=150.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the latents the last timed inversion step and edit step returned (rank 0) "
+                         "as DIR/inversion_latents.npy and DIR/edit_latents.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm only times the oracle")
     global F
     F = args.frames
     if args.warmup < 4:

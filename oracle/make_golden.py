@@ -13,6 +13,7 @@ What is pinned here (the reference has no tests; diffusers is absent — see ora
 from __future__ import annotations
 
 import os
+import shutil
 from types import SimpleNamespace
 
 import torch
@@ -92,6 +93,12 @@ def main():
             kat[f"inv_step_{n}_{t}"] = a.clone()
     torch.save(kat, os.path.join(OUT, "scheduler_kat.pt"))
     print("scheduler: vendored reference class == restatement (alphas, timesteps, inverse step) — bit-exact")
+
+    # ---- the reference's config templates, verbatim, for the config API test
+    for rel in ("group_pnp_edit/template.yaml", "group_pnp_edit/group_config.json", "group_ddim_inversion/template.yaml"):
+        dst = os.path.join(OUT, "reference_configs", rel)
+        os.makedirs(os.path.dirname(dst), exist_ok=True)
+        shutil.copyfile(os.path.join(diffusers_shim.REF_ROOT, "i2vgen-xl", "configs", rel), dst)
     for f in sorted(os.listdir(OUT)):
         print(f"  tests/golden/{f}: {os.path.getsize(os.path.join(OUT, f))} bytes")
 

@@ -42,10 +42,10 @@ def test_ops_refuse_cpu_tensors_loudly():
         ops.groupnorm(torch.zeros(1, 4, 32, dtype=torch.float16), torch.ones(32).half(), torch.zeros(32).half(), 32, 1e-5, True)
 
 
-REF_CFG = "/root/reference/i2vgen-xl/configs"
+# the reference's own i2vgen-xl/configs templates (and group_pnp_edit's group_config.json), stored verbatim (oracle/make_golden.py)
+REF_CFG = os.path.join(ROOT, "tests", "golden", "reference_configs")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CFG), reason="reference configs only exist in the build container")
 def test_config_api_on_the_reference_templates():
     from anyv2v_b200.config import OmegaConf
     t = OmegaConf.load(f"{REF_CFG}/group_pnp_edit/template.yaml")
@@ -255,6 +255,23 @@ def test_bench_cpu_arm_thread_budget_respects_the_cgroup_quota(monkeypatch):
         assert n <= len(os.sched_getaffinity(0))
     except AttributeError:
         pass
+
+
+def test_bench_dump_outputs_float32_within_budget_same_sample(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: float32 .npy files, an array over its share of the byte budget replaced by the same seeded sample
+    of its elements in every run."""
+    import numpy as np
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4000)
+    g = torch.Generator().manual_seed(3)
+    big, small = torch.randn(1, 4, 16, 8, 8, generator=g).half().float(), torch.randn(2, 3, generator=g)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"big": big, "small": small})
+    got = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("big", "small")}
+    assert all(v.dtype == np.float32 for v in got.values()) and sum(v.nbytes for v in got.values()) <= 4000
+    np.testing.assert_array_equal(got["small"], small.numpy())
+    assert got["big"].shape == (500,) and np.isin(got["big"], big.numpy()).all()
+    np.testing.assert_array_equal(np.load(tmp_path / "b" / "big.npy"), got["big"])
 
 
 def test_bench_roofline_traffic_comes_from_the_committed_ncu_extracts():
