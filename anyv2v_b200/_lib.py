@@ -38,6 +38,11 @@ class GemmArgs(Structure):
                 ("a2", c_void_p), ("k_split", c_int32), ("lda2", c_int32), ("up2_phase", c_int32)]
 
 
+class ConvPlan(Structure):
+    _fields_ = [("box_w", c_int32), ("box_h", c_int32), ("frames_per_tile", c_int32), ("tiles_per_frame", c_int32),
+                ("m_tiles", c_int32)]
+
+
 class LayerNormArgs(Structure):
     _fields_ = [("x", c_void_p), ("y", c_void_p), ("gamma", c_void_p), ("beta", c_void_p), ("rows", c_int64),
                 ("C", c_int32), ("eps", c_float)]
@@ -66,6 +71,7 @@ EXPORTS = {
     "av2v_groupnorm_workspace_floats": (c_int, [c_int, c_int]),
     "av2v_groupnorm_silu_f16": (c_int, [POINTER(GroupNormArgs), c_void_p]),
     "av2v_gemm_f16": (c_int, [POINTER(GemmArgs), c_void_p]),
+    "av2v_conv3x3_plan": (c_int, [POINTER(GemmArgs), POINTER(ConvPlan)]),
     "av2v_layernorm_f16": (c_int, [POINTER(LayerNormArgs), c_void_p]),
     "av2v_attn_pnp_f16": (c_int, [POINTER(AttnArgs), c_void_p]),
     "av2v_tattn_fused_f16": (c_int, [POINTER(TAttnFusedArgs), c_void_p]),

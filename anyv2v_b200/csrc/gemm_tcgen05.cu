@@ -7,13 +7,15 @@
 //   warp 1  : MMA issuer    (one lane issues tcgen05.mma 128 x BN x 16, fp32 accumulators in TMEM, double-buffered)
 //   warp 2  : TMEM allocator
 //   warps 4-11: epilogue    (two warpgroups on alternate 32-column chunks: tcgen05.ld -> +bias/+rowbias/+residual -> fp16 ->
-//                            swizzled smem -> bulk TMA store, 1..n_slots copies; direct 16 B stores when a tile's rows are not
-//                            contiguous in the output).  The epilogue is a template parameter: three lean straight-line flavours
+//                            swizzled smem -> bulk TMA store, 1..n_slots copies; a conv tile that is a block of pixels goes
+//                            through a 5-D (c, x, y, frame, slot) map that clips it at the image edges; direct 16 B stores for
+//                            temporal-conv tiles whose rows are not contiguous in the output).  The epilogue is a template parameter: three lean straight-line flavours
 //                            (plain / +residual / GEGLU, one slot) and the generic one — for short K the epilogue warps' instruction
 //                            stream, not the tensor pipe, sets the tile time (profiles/r02_gemm_k320_epilogue.txt)
 //
 // The A operand is never materialised as an im2col buffer: for 3x3 convolutions the producer issues one 4-D TMA
-// box per filter tap with the (dy, dx) shift folded into the coordinates (out-of-bounds = zero padding); for the
+// box per filter tap with the (dy, dx) shift folded into the coordinates (out-of-bounds = zero padding; the box is the tile's
+// block of box_h x box_w output pixels, or whole frames — av2v_conv3x3_plan); for the
 // (3,1,1) temporal convolution a 3-D box shifted by +-HW rows within the clip.
 //
 // Replaces (reference = library calls inside PyTorch): cuBLAS Linear at pnp_utils.py:178-186,216; cuDNN conv at
@@ -40,16 +42,18 @@ constexpr int kNumOutBufs = 3;           // per group: output staging ring (TMA 
 constexpr int kRes = 2;
 
 // epilogue flavours (template parameter): the generic one covers every combination (slots, row bias, up-sampling store, GEGLU,
-// residual, direct stores); the lean ones are straight-line code for the three shapes the short-K projections use
-enum { E_GENERIC = 0, E_PLAIN = 1, E_RES = 2, E_GEGLU = 3 };
+// residual, direct stores); the lean ones are straight-line code for the three shapes the short-K projections use.  E_BLOCK (a flag
+// on E_PLAIN / E_RES): the conv tiles are pixel blocks stored through the 5-D block map — a separate instantiation, so that the
+// row-contiguous lean kernels the projections run carry none of the block bookkeeping
+enum { E_GENERIC = 0, E_PLAIN = 1, E_RES = 2, E_GEGLU = 3, E_BLOCK = 4 };
 
 template <int BN, bool kPair, int kEpi>
 struct GemmCfg {
   // ... and two output staging buffers per group are enough for the lean flavours (the store of chunk n - 1 has one chunk time to
   // read its source): +1 pipeline stage for most tile shapes (measured: 196608x960x320 147.7 -> 131.7 us, GEGLU 12288x10240x1280 213.8 -> 202.7)
-  static constexpr int kOutBufs = (kEpi != E_GENERIC) ? 2 : kNumOutBufs;
+  static constexpr int kOutBufs = ((kEpi & 3) != E_GENERIC) ? 2 : kNumOutBufs;
   // the plain and GEGLU flavours never stage a residual: their two buffers per group become (part of) one more pipeline stage
-  static constexpr int kResBufs = (kEpi == E_PLAIN || kEpi == E_GEGLU) ? 0 : kRes;
+  static constexpr int kResBufs = ((kEpi & 3) == E_PLAIN || (kEpi & 3) == E_GEGLU) ? 0 : kRes;
   static constexpr int kEpiBytes = kEpiGroups * (kOutBufs + kResBufs) * kEpiBufBytes;
   static constexpr int kABytes = BM * BK * 2;
   static constexpr int kBBytes = (kPair ? BN / 2 : BN) * BK * 2;  // pair mode: each CTA stages only its half of the W tile
@@ -70,13 +74,18 @@ struct GemmKParams {
   int num_kb, kb_per_tap;
   int mode;
   int m_tiles, n_tiles;
-  // conv3x3 geometry
-  int H, W, HW, NF, box_h, tiles_per_frame, frames_per_tile;
-  int x_tiles;  // W > 128: a tile is a 128-pixel segment of one image row, x_tiles = W / 128 segments per row (else 1)
+  // conv3x3 geometry: a tile is a block of box_h rows x box_w columns of one frame (x_tiles = ceil(W / box_w) blocks per row of
+  // blocks), or frames_per_tile > 1 whole frames; tile order (frame, row block, column block) — av2v_conv3x3_plan
+  int H, W, HW, NF, box_w, box_h, tiles_per_frame, frames_per_tile;
+  int x_tiles;
+  int block_store;  // conv3x3: the tile's rows are not 128 consecutive output rows -> stores / residual loads through the 5-D
+                    // block map (c, x, y, frame, slot), which clips the block at the image's right and bottom edges
+  uint32_t o_box_bytes;  // bytes of one 32-column staging chunk as the store / residual map moves it (64 B per tile row)
   int stride;   // conv3x3: 1 or 2 (H, W above are the OUTPUT geometry; the taps address input pixel stride * out + tap - 1)
   int taps_w;   // 3: 3 x 3 taps at offsets -1 .. +1; 2: the 2 x 2 taps of one output phase of "nearest-up x 2 then conv 3 x 3"
   int tap_oy, tap_ox;  // taps_w = 2: phase (py, px): tap (a, b) reads input pixel (i + a - 1 + py, j + b - 1 + px)
   int up2;      // 1: the tile's pixels (i, j) are stored to output pixels (2 i + py, 2 j + px) through a 5-D tensor map
+                //    (px * N + c, j, py, i, frame)
   int kb_split; // linear: k-blocks [0, kb_split) come from tmap_a, the rest from tmap_a2 (two-source K loop); = num_kb otherwise
   // tconv geometry
   int tiles_per_clip, rows_per_clip;
@@ -111,6 +120,22 @@ struct TileSched {
     return true;
   }
 };
+
+// conv3x3: first output pixel (frame n0, row y0, column x0) of tile m_tile; tile row r of the accumulator is pixel
+// (n0 + r / (box_w * box_h), y0 + (r / box_w) % box_h, x0 + r % box_w) — the order of the A box in shared memory
+__device__ __forceinline__ void conv_tile_origin(const GemmKParams& p, int m_tile, int& n0, int& y0, int& x0) {
+  if (p.frames_per_tile == 1) {
+    n0 = m_tile / p.tiles_per_frame;
+    const int rem = m_tile - n0 * p.tiles_per_frame;
+    const int yb = rem / p.x_tiles;
+    y0 = yb * p.box_h;
+    x0 = (rem - yb * p.x_tiles) * p.box_w;
+  } else {
+    n0 = m_tile * p.frames_per_tile;
+    y0 = 0;
+    x0 = 0;
+  }
+}
 
 // Exact-erf GELU, branch-free: gelu(g) = g/2 + |g|/2 * erf(|g|/sqrt 2) with erf from Abramowitz & Stegun 7.1.25
 // (3-term, |abs err| < 2.5e-5 — two orders below fp16 resolution) on MUFU rcp / ex2: ~14 instructions per element.
@@ -239,16 +264,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
       for (int ti = 0; sched.get(ti, m_tile, n_tile); ++ti) {
         int c_n = 0, c_y = 0, c_r = 0, c_x = 0;
         if (p.mode == AV2V_A_CONV3X3) {
-          if (p.frames_per_tile == 1) {
-            c_n = m_tile / p.tiles_per_frame;
-            const int rem = m_tile - c_n * p.tiles_per_frame;
-            const int yb = rem / p.x_tiles;
-            c_y = yb * p.box_h;
-            c_x = (rem - yb * p.x_tiles) * BM;
-          } else {
-            c_n = m_tile * p.frames_per_tile;
-            c_y = 0;
-          }
+          conv_tile_origin(p, m_tile, c_n, c_y, c_x);
         } else if (p.mode == AV2V_A_TCONV3) {
           c_n = m_tile / p.tiles_per_clip;
           c_r = (m_tile - c_n * p.tiles_per_clip) * BM;
@@ -363,13 +379,13 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
     const int q = warp & 3;
     const int r = q * 32 + lane;
     uint32_t it = 0;
-    if constexpr (kEpi != E_GENERIC) {
+    if constexpr ((kEpi & 3) != E_GENERIC) {
       // ---- lean staged epilogue (one output slot, no up-sampling store): the flavour is a template parameter, so
       // the per-chunk code is one straight line.  Why: for K = 320 the tile time is set by the epilogue warps, two per
       // scheduler, whose time is their instruction count times the exposed latency (and an instruction-fetch stall after every
       // taken branch over the generic path's cold code) — profiles/r02_gemm_k320_epilogue.txt.  Tile coordinates advance
       // incrementally (no divisions), ring indices are counters, the bias is fp32 in shared memory (packed fp32x2 adds).
-      constexpr bool kWithRes = (kEpi == E_RES), kGeglu = (kEpi == E_GEGLU);
+      constexpr bool kWithRes = ((kEpi & 3) == E_RES), kGeglu = ((kEpi & 3) == E_GEGLU), kBlock = (kEpi & E_BLOCK) != 0;
       constexpr int kStep = kGeglu ? 4 : 2, kLog = kGeglu ? 2 : 1;
       const int eg = (warp - 4) >> 2;                         // epilogue group 0 / 1
       const uint32_t el = elect_one() ? 1u : 0u;              // this warp's issuing lane, when it is the warp's turn
@@ -382,6 +398,15 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
       uint32_t soff[4];
 #pragma unroll
       for (int j4 = 0; j4 < 4; ++j4) soff[j4] = r * 64 + ((j4 ^ swz) << 4);
+      // block-shaped conv tiles: this thread's row is pixel (bz, by, bx) of the block (fixed); the block's origin is derived from
+      // m_tile once per tile (divisions by runtime constants — only on this path)
+      int bx = 0, by = 0, bz = 0;
+      if constexpr (kBlock) {
+        const int bwh = p.box_w * p.box_h;
+        bz = r / bwh;
+        by = (r - bz * bwh) / p.box_w;
+        bx = r - bz * bwh - by * p.box_w;
+      }
       // tile iterator: unit u = first + i * stride -> (mu, n_tile), advanced without divisions
       const int nt = sched.n_tiles;
       const int dm = sched.stride / nt, dn = sched.stride - dm * nt;
@@ -409,8 +434,15 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
         }
         if (pf_mu >= mu_count) return;
         const uint32_t bar = u_resbar + pf_buf * 8, dst = u_res + pf_buf * kEpiBufBytes;
-        mbar_arrive_expect_tx_w(issue, bar, kEpiBufBytes);
-        tma_load_3d_w(issue, dst, &tmap_r, bar, pf_n * BN + pf_c * 32, (sched.mc2 ? 2 * pf_mu + sched.rank : pf_mu) * BM, 0);
+        const int pf_m = sched.mc2 ? 2 * pf_mu + sched.rank : pf_mu;
+        mbar_arrive_expect_tx_w(issue, bar, kBlock ? p.o_box_bytes : static_cast<uint32_t>(kEpiBufBytes));
+        if constexpr (kBlock) {
+          int n0, y0, x0;
+          conv_tile_origin(p, pf_m, n0, y0, x0);
+          tma_load_5d_w(issue, dst, &tmap_r, bar, pf_n * BN + pf_c * 32, x0, y0, n0, 0);
+        } else {
+          tma_load_3d_w(issue, dst, &tmap_r, bar, pf_n * BN + pf_c * 32, pf_m * BM, 0);
+        }
         pf_buf ^= 1u;
         pf_c += kStep;
       };
@@ -428,8 +460,15 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
         const uint32_t acc = it & 1u;
         const uint32_t acc_phase = (it >> 1) & 1u;
         const int nchunks = AV2V_DBG(16) ? 0 : chunks_of(n_tile);
-        const long long grow = static_cast<long long>(m_tile) * BM + r;  // staged tiles: 128 consecutive output rows
-        const bool valid = grow < p.M;
+        long long grow = static_cast<long long>(m_tile) * BM + r;  // contiguous tiles: 128 consecutive output rows
+        bool valid = grow < p.M;
+        int o_x = 0, o_y = m_tile * BM, o_n = 0;  // store / residual coordinates of the tile (contiguous: row, -)
+        if constexpr (kBlock) {
+          conv_tile_origin(p, m_tile, o_n, o_y, o_x);
+          const int xx = o_x + bx, yy = o_y + by, nn = o_n + bz;
+          valid = bz < p.frames_per_tile && xx < p.W && yy < p.H && nn < p.NF;
+          grow = static_cast<long long>(nn) * p.HW + static_cast<long long>(yy) * p.W + xx;
+        }
         const int rb_row = (p.rowbias != nullptr && valid) ? static_cast<int>(grow / p.rows_per_rowbias) : 0;
         const int first = kGeglu ? 2 * eg : (eg ^ par);
         const int n_own = nchunks > first ? (nchunks - first + kStep - 1) >> kLog : 0;
@@ -546,8 +585,12 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
           asm volatile("bar.sync %0, 128;" ::"r"(1 + eg) : "memory");
           const uint32_t issue = (q == static_cast<int>(turn)) ? el : 0u;
           if (q == static_cast<int>(turn) && !AV2V_DBG(64)) {
-            tma_store_3d_w(issue, &tmap_o, __shfl_sync(0xffffffffu, obuf, 0), __shfl_sync(0xffffffffu, col0, 0),
-                           __shfl_sync(0xffffffffu, m_tile * BM, 0), 0);
+            if constexpr (kBlock)
+              tma_store_5d_w(issue, &tmap_o, __shfl_sync(0xffffffffu, obuf, 0), __shfl_sync(0xffffffffu, col0, 0),
+                             __shfl_sync(0xffffffffu, o_x, 0), __shfl_sync(0xffffffffu, o_y, 0), __shfl_sync(0xffffffffu, o_n, 0), 0);
+            else
+              tma_store_3d_w(issue, &tmap_o, __shfl_sync(0xffffffffu, obuf, 0), __shfl_sync(0xffffffffu, col0, 0),
+                             __shfl_sync(0xffffffffu, o_y, 0), 0);
             if (issue) tma_store_commit();
             __syncwarp();
           }
@@ -587,6 +630,13 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
       for (int j4 = 0; j4 < 4; ++j4) soff[j4] = r * 64 + ((j4 ^ swz) << 4);
       uint64_t* my_res_full = res_full + eg * kNumResBufs;
       float* my_bias = bias_stage + eg * 128;                  // fp32 bias of the (up to four) chunks this group owns in a tile
+      int bx = 0, by = 0, bz = 0;                              // block-shaped conv tiles: this thread's pixel within the block
+      if (p.block_store) {
+        const int bwh = p.box_w * p.box_h;
+        bz = r / bwh;
+        by = (r - bz * bwh) / p.box_w;
+        bx = r - bz * bwh - by * p.box_w;
+      }
       const int step = p.geglu ? 4 : 2;                        // chunk stride between this group's work units
       auto first_of = [&](int ti) { return p.geglu ? 2 * eg : (eg ^ (ti & 1)); };  // first chunk of this group in tile ti
       auto chunks_of = [&](int n_tile) {
@@ -611,9 +661,16 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
         const uint32_t b = pf_iter % kNumResBufs;
         const uint32_t u_bar = __shfl_sync(0xffffffffu, smem_u32(&my_res_full[b]), 0);
         const uint32_t u_dst = __shfl_sync(0xffffffffu, u_res + b * kEpiBufBytes, 0);
-        mbar_arrive_expect_tx_w(issue, u_bar, kEpiBufBytes);
-        tma_load_3d_w(issue, u_dst, &tmap_r, u_bar, __shfl_sync(0xffffffffu, pf_n * BN + pf_c * 32, 0),
-                      __shfl_sync(0xffffffffu, pf_m * BM, 0), __shfl_sync(0xffffffffu, pf_s, 0));
+        mbar_arrive_expect_tx_w(issue, u_bar, p.o_box_bytes);
+        if (p.block_store) {
+          int n0, y0, x0;
+          conv_tile_origin(p, pf_m, n0, y0, x0);
+          tma_load_5d_w(issue, u_dst, &tmap_r, u_bar, __shfl_sync(0xffffffffu, pf_n * BN + pf_c * 32, 0), __shfl_sync(0xffffffffu, x0, 0),
+                        __shfl_sync(0xffffffffu, y0, 0), __shfl_sync(0xffffffffu, n0, 0), __shfl_sync(0xffffffffu, pf_s, 0));
+        } else {
+          tma_load_3d_w(issue, u_dst, &tmap_r, u_bar, __shfl_sync(0xffffffffu, pf_n * BN + pf_c * 32, 0),
+                        __shfl_sync(0xffffffffu, pf_m * BM, 0), __shfl_sync(0xffffffffu, pf_s, 0));
+        }
         ++pf_iter;
         if (++pf_s == p.n_slots) {
           pf_s = 0;
@@ -628,8 +685,15 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
       for (int ti = 0; sched.get(ti, m_tile, n_tile); ++ti, ++it) {
         const uint32_t acc = it & 1u;
         const uint32_t acc_phase = (it >> 1) & 1u;
-        const long long grow = static_cast<long long>(m_tile) * BM + r;
-        const bool valid = grow < p.M;
+        long long grow = static_cast<long long>(m_tile) * BM + r;
+        bool valid = grow < p.M;
+        int o_n = 0, o_y = 0, o_x = 0;  // block stores / up2: the tile's first output pixel
+        if (p.block_store || p.up2) conv_tile_origin(p, m_tile, o_n, o_y, o_x);
+        if (p.block_store) {
+          const int xx = o_x + bx, yy = o_y + by, nn = o_n + bz;
+          valid = bz < p.frames_per_tile && xx < p.W && yy < p.H && nn < p.NF;
+          grow = static_cast<long long>(nn) * p.HW + static_cast<long long>(yy) * p.W + xx;
+        }
         const long long rb_row = (p.rowbias != nullptr && valid) ? grow / p.rows_per_rowbias : 0;
         const int nchunks = AV2V_DBG(16) ? 0 : chunks_of(n_tile);  // bring-up: bit4 = epilogue only frees the accumulator
         const int first = first_of(ti);
@@ -758,8 +822,11 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
               // operands made provably warp-uniform (shfl) so that the store is issued from uniform registers
               const uint32_t u_src = __shfl_sync(0xffffffffu, obuf, 0);
               const int u_c0 = __shfl_sync(0xffffffffu, col0, 0), u_c1 = __shfl_sync(0xffffffffu, m_tile * BM, 0);
-              if (p.up2)  // rows of the tile = (global input row I, column j); output pixel (2 I + py, 2 j + px)
-                tma_store_5d_w(issue, &tmap_o, u_src, u_c0, p.tap_ox, 0, p.tap_oy, u_c1 / p.W);
+              const int u_x = __shfl_sync(0xffffffffu, o_x, 0), u_y = __shfl_sync(0xffffffffu, o_y, 0), u_n = __shfl_sync(0xffffffffu, o_n, 0);
+              if (p.up2)  // tile pixel (n, i, j) -> output pixel (n, 2 i + py, 2 j + px)
+                tma_store_5d_w(issue, &tmap_o, u_src, u_c0 + p.tap_ox * p.N, u_x, p.tap_oy, u_y, u_n);
+              else if (p.block_store)
+                tma_store_5d_w(issue, &tmap_o, u_src, u_c0, u_x, u_y, u_n, __shfl_sync(0xffffffffu, s, 0));
               else
                 tma_store_3d_w(issue, &tmap_o, u_src, u_c0, u_c1, __shfl_sync(0xffffffffu, s, 0));
               if (issue) tma_store_commit();
@@ -777,20 +844,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
 
       long long grow;
       bool valid;
-      if (p.mode == AV2V_A_CONV3X3) {
-        if (p.frames_per_tile == 1) {
-          const int n = m_tile / p.tiles_per_frame;
-          const int y0 = (m_tile - n * p.tiles_per_frame) * p.box_h;
-          const int yy = r / p.W;
-          valid = (r < p.box_h * p.W) && (y0 + yy < p.H);
-          grow = static_cast<long long>(n) * p.HW + static_cast<long long>(y0) * p.W + r;
-        } else {
-          const int n0 = m_tile * p.frames_per_tile;
-          const int nn = r / p.HW;
-          valid = (nn < p.frames_per_tile) && (n0 + nn < p.NF);
-          grow = static_cast<long long>(n0) * p.HW + r;
-        }
-      } else if (p.mode == AV2V_A_TCONV3) {
+      if (p.mode == AV2V_A_TCONV3) {  // (conv3x3 tiles always take the staged epilogue through the block map)
         const int b = m_tile / p.tiles_per_clip;
         const int r0 = (m_tile - b * p.tiles_per_clip) * BM;
         valid = (r0 + r) < p.rows_per_clip;
@@ -928,7 +982,7 @@ int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap&
 #else
   const bool lean = p.fast_epi && p.n_slots == 1 && !p.up2;
 #endif
-  const int epi = !lean ? E_GENERIC : p.geglu ? E_GEGLU : p.residual != nullptr ? E_RES : E_PLAIN;
+  const int epi = !lean ? E_GENERIC : p.geglu ? E_GEGLU : (p.residual != nullptr ? E_RES : E_PLAIN) | (p.block_store ? E_BLOCK : 0);
 #define AV2V_LAUNCH(E)                                                                              \
   return p.mc2 == 2 ? launch_gemm_impl<BN, true, E>(ta, tb, to, tr, tbh, ta2, p, stream)           \
                     : launch_gemm_impl<BN, false, E>(ta, tb, to, tr, tbh, ta2, p, stream)
@@ -936,6 +990,8 @@ int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap&
     case E_PLAIN: AV2V_LAUNCH(E_PLAIN);
     case E_RES: AV2V_LAUNCH(E_RES);
     case E_GEGLU: AV2V_LAUNCH(E_GEGLU);
+    case E_PLAIN | E_BLOCK: AV2V_LAUNCH(E_PLAIN | E_BLOCK);
+    case E_RES | E_BLOCK: AV2V_LAUNCH(E_RES | E_BLOCK);
     default: AV2V_LAUNCH(E_GENERIC);
   }
 #undef AV2V_LAUNCH
@@ -948,6 +1004,65 @@ using namespace av2v;
 
 extern "C" int av2v_gemm_debug_timers(unsigned long long* out16) {
   AV2V_CHECK_CUDA(cudaMemcpyFromSymbol(out16, av2v::g_gemm_timers, sizeof(unsigned long long) * 16));
+  return AV2V_OK;
+}
+
+// Validation and tile plan of a CONV3X3 call (host only).  Frames of at most 64 pixels: several whole frames per tile.  Widths
+// that divide 128: whole image rows.  Any other width: the block of box_w x box_h pixels (box_w in {128, 64, 32, 16, 8, W_out},
+// box_h = 128 / box_w) with the fewest tiles per frame, the wider block on a tie — 128-pixel row segments for widths that are
+// multiples of 128, e.g. 32 x 4 at 160 x 88 and 8 x 16 at 88 x 160 (both fill every tile).
+extern "C" int av2v_conv3x3_plan(const av2v_gemm_args* a, av2v_conv_plan* out) {
+  AV2V_REQUIRE(a != nullptr && out != nullptr, AV2V_EINVAL, "conv3x3 plan: null args");
+  AV2V_REQUIRE(a->mode == AV2V_A_CONV3X3, AV2V_EINVAL, "conv3x3 plan: mode must be AV2V_A_CONV3X3 (got %d)", a->mode);
+  AV2V_REQUIRE(a->NF > 0 && a->H > 0 && a->W > 0 && a->Cin > 0, AV2V_EINVAL, "gemm/conv3x3: bad geometry");
+  AV2V_REQUIRE(a->Cin % BK == 0, AV2V_ENOSUP, "gemm/conv3x3: Cin must be a multiple of 64 (got %d)", a->Cin);
+  const int up = a->up2_phase;  // 0: plain conv; 1..4: phase (py, px) = ((up-1) >> 1, (up-1) & 1) of nearest-up x 2 + conv 3 x 3
+  AV2V_REQUIRE(up >= 0 && up <= 4, AV2V_EINVAL, "gemm/conv3x3: up2_phase must be 0..4 (got %d)", up);
+  AV2V_REQUIRE(a->K == (up ? 4 : 9) * a->Cin, AV2V_EINVAL, "gemm/conv3x3: K must equal 9*Cin (4*Cin for an up2 phase)");
+  AV2V_REQUIRE(!up || (a->stride <= 1 && !a->rowbias && !a->residual && a->n_slots == 1), AV2V_EINVAL,
+               "gemm/conv3x3: an up2 phase takes bias only (no stride, rowbias, residual, slots)");
+  // the up2 store map merges (px, channel) into one dimension of 2 N contiguous channels; 32-column chunks must not straddle px
+  AV2V_REQUIRE(!up || (a->ldo == a->N && a->N % 32 == 0), AV2V_ENOSUP,
+               "gemm/conv3x3 up2: needs a contiguous output (ldo == N) and N a multiple of 32 (N = %d, ldo = %d)", a->N, a->ldo);
+  const int stride = a->stride == 0 ? 1 : a->stride;
+  AV2V_REQUIRE(stride == 1 || stride == 2, AV2V_ENOSUP, "gemm/conv3x3: stride must be 1 or 2 (got %d)", a->stride);
+  AV2V_REQUIRE(a->H % stride == 0 && a->W % stride == 0, AV2V_ENOSUP, "gemm/conv3x3: H, W must be multiples of the stride");
+  const int chan = a->a_channels == 0 ? a->Cin : a->a_channels;
+  AV2V_REQUIRE(chan > 0 && chan <= a->Cin && chan % 8 == 0, AV2V_EINVAL, "gemm/conv3x3: a_channels must be a multiple of 8 in (0, Cin]");
+  const int Ho = a->H / stride, Wo = a->W / stride;  // output geometry: the plan tiles the OUTPUT pixels
+  AV2V_REQUIRE(static_cast<long long>(a->NF) * Ho * Wo == a->M, AV2V_EINVAL, "gemm/conv3x3: M != NF*(H/stride)*(W/stride)");
+  const long long HW = static_cast<long long>(Ho) * Wo;
+  av2v_conv_plan pl{};
+  if (2 * HW <= BM) {  // several whole frames per tile
+    pl.box_w = Wo;
+    pl.box_h = Ho;
+    pl.frames_per_tile = static_cast<int>(BM / HW);
+    pl.tiles_per_frame = 1;
+    pl.m_tiles = (a->NF + pl.frames_per_tile - 1) / pl.frames_per_tile;
+  } else {
+    pl.frames_per_tile = 1;
+    if (Wo <= BM && BM % Wo == 0) {  // whole image rows
+      pl.box_w = Wo;
+      pl.box_h = BM / Wo < Ho ? BM / Wo : Ho;
+    } else {
+      const int cands[6] = {BM, 64, 32, 16, 8, Wo < BM ? Wo : 0};
+      long long best = -1;
+      for (int i = 0; i < 6; ++i) {
+        const int bw = cands[i];
+        if (bw == 0) continue;
+        const int bh = BM / bw < Ho ? BM / bw : Ho;
+        const long long tiles = static_cast<long long>((Wo + bw - 1) / bw) * ((Ho + bh - 1) / bh);
+        if (best < 0 || tiles < best || (tiles == best && bw > pl.box_w)) {  // fewest tiles, then the wider block
+          best = tiles;
+          pl.box_w = bw;
+          pl.box_h = bh;
+        }
+      }
+    }
+    pl.tiles_per_frame = ((Wo + pl.box_w - 1) / pl.box_w) * ((Ho + pl.box_h - 1) / pl.box_h);
+    pl.m_tiles = a->NF * pl.tiles_per_frame;
+  }
+  *out = pl;
   return AV2V_OK;
 }
 
@@ -1028,13 +1143,9 @@ extern "C" int av2v_gemm_f16(const av2v_gemm_args* a, av2v_stream_t stream_) {
       p.kb_split = a->k_split / BK;
     }
   } else if (a->mode == AV2V_A_CONV3X3) {
-    AV2V_REQUIRE(a->NF > 0 && a->H > 0 && a->W > 0 && a->Cin > 0, AV2V_EINVAL, "gemm/conv3x3: bad geometry");
-    AV2V_REQUIRE(a->Cin % BK == 0, AV2V_ENOSUP, "gemm/conv3x3: Cin must be a multiple of 64 (got %d)", a->Cin);
-    const int up = a->up2_phase;  // 0: plain conv; 1..4: phase (py, px) = ((up-1) >> 1, (up-1) & 1) of nearest-up x 2 + conv 3 x 3
-    AV2V_REQUIRE(up >= 0 && up <= 4, AV2V_EINVAL, "gemm/conv3x3: up2_phase must be 0..4 (got %d)", up);
-    AV2V_REQUIRE(a->K == (up ? 4 : 9) * a->Cin, AV2V_EINVAL, "gemm/conv3x3: K must equal 9*Cin (4*Cin for an up2 phase)");
-    AV2V_REQUIRE(!up || (a->stride <= 1 && !a->rowbias && !a->residual && a->n_slots == 1), AV2V_EINVAL,
-                 "gemm/conv3x3: an up2 phase takes bias only (no stride, rowbias, residual, slots)");
+    av2v_conv_plan pl;
+    if ((rc = av2v_conv3x3_plan(a, &pl)) != AV2V_OK) return rc;
+    const int up = a->up2_phase;
     if (up) {
       p.taps_w = 2;
       p.tap_oy = (up - 1) >> 1;
@@ -1042,53 +1153,32 @@ extern "C" int av2v_gemm_f16(const av2v_gemm_args* a, av2v_stream_t stream_) {
       p.up2 = 1;
     }
     const int stride = a->stride == 0 ? 1 : a->stride;
-    AV2V_REQUIRE(stride == 1 || stride == 2, AV2V_ENOSUP, "gemm/conv3x3: stride must be 1 or 2 (got %d)", a->stride);
-    AV2V_REQUIRE(a->H % stride == 0 && a->W % stride == 0, AV2V_ENOSUP, "gemm/conv3x3: H, W must be multiples of the stride");
     const int chan = a->a_channels == 0 ? a->Cin : a->a_channels;  // channels really present (the rest of the K block reads zeros)
-    AV2V_REQUIRE(chan > 0 && chan <= a->Cin && chan % 8 == 0, AV2V_EINVAL, "gemm/conv3x3: a_channels must be a multiple of 8 in (0, Cin]");
-    const int Ho = a->H / stride, Wo = a->W / stride;  // output geometry: everything below tiles the OUTPUT pixels
-    AV2V_REQUIRE(static_cast<long long>(a->NF) * Ho * Wo == a->M, AV2V_EINVAL, "gemm/conv3x3: M != NF*(H/stride)*(W/stride)");
-    AV2V_REQUIRE(Wo <= BM || Wo % BM == 0, AV2V_ENOSUP,
-                 "gemm/conv3x3: output width must be <= 128 or a multiple of 128 (got %d)", Wo);
-    AV2V_REQUIRE(stride == 1 || Wo <= BM, AV2V_ENOSUP, "gemm/conv3x3: stride 2 needs an output width <= 128");
+    const int Ho = a->H / stride, Wo = a->W / stride;
     p.stride = stride;
     p.H = Ho;
     p.W = Wo;
     p.HW = Ho * Wo;
     p.NF = a->NF;
-    p.x_tiles = 1;
-    uint32_t box_w = static_cast<uint32_t>(Wo);
-    if (Wo > BM) {  // wide images (VAE resolutions): one tile = a 128-pixel segment of one row
-      p.frames_per_tile = 1;
-      p.box_h = 1;
-      p.x_tiles = Wo / BM;
-      p.tiles_per_frame = Ho * p.x_tiles;
-      p.m_tiles = a->NF * p.tiles_per_frame;
-      box_w = BM;
-    } else if (p.HW >= BM || BM / p.HW < 2) {
-      p.frames_per_tile = 1;
-      p.box_h = BM / Wo;
-      if (p.box_h > Ho) p.box_h = Ho;
-      p.tiles_per_frame = (Ho + p.box_h - 1) / p.box_h;
-      p.m_tiles = a->NF * p.tiles_per_frame;
-    } else {
-      p.frames_per_tile = BM / p.HW;
-      p.box_h = Ho;
-      p.tiles_per_frame = 1;
-      p.m_tiles = (a->NF + p.frames_per_tile - 1) / p.frames_per_tile;
-    }
+    p.box_w = pl.box_w;
+    p.box_h = pl.box_h;
+    p.frames_per_tile = pl.frames_per_tile;
+    p.tiles_per_frame = pl.tiles_per_frame;
+    p.x_tiles = (Wo + pl.box_w - 1) / pl.box_w;
+    p.m_tiles = pl.m_tiles;
     // the tensor map describes the INPUT image; with stride 2 the box spans 2x the output pixels and TMA picks every second one
     const uint64_t dims[4] = {static_cast<uint64_t>(chan), static_cast<uint64_t>(a->W),
                               static_cast<uint64_t>(a->H), static_cast<uint64_t>(a->NF)};
     const uint64_t str[3] = {static_cast<uint64_t>(chan) * 2, static_cast<uint64_t>(chan) * 2 * a->W,
                              static_cast<uint64_t>(chan) * 2 * a->W * a->H};
-    const uint32_t box[4] = {BK, box_w * stride, static_cast<uint32_t>(p.box_h) * stride, static_cast<uint32_t>(p.frames_per_tile)};
+    const uint32_t box[4] = {BK, static_cast<uint32_t>(pl.box_w * stride), static_cast<uint32_t>(pl.box_h * stride),
+                             static_cast<uint32_t>(pl.frames_per_tile)};
     const uint32_t estr[4] = {1, static_cast<uint32_t>(stride), static_cast<uint32_t>(stride), 1};
     if ((rc = make_tmap_f16(&ta, a->a, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B, estr)) != AV2V_OK) return rc;
     p.kb_per_tap = a->Cin / BK;
     p.num_kb = (up ? 4 : 9) * p.kb_per_tap;
     p.kb_split = p.num_kb;
-    p.a_box_bytes = static_cast<uint32_t>(BK * 2 * box_w * p.box_h * p.frames_per_tile);
+    p.a_box_bytes = static_cast<uint32_t>(BK * 2 * pl.box_w * pl.box_h * pl.frames_per_tile);  // < 128 rows: the rest is never stored
   } else if (a->mode == AV2V_A_TCONV3) {
     AV2V_REQUIRE(a->B > 0 && a->rows_per_clip > 0 && a->HW > 0 && a->Cin > 0, AV2V_EINVAL, "gemm/tconv3: bad geometry");
     AV2V_REQUIRE(a->Cin % BK == 0, AV2V_ENOSUP, "gemm/tconv3: Cin must be a multiple of 64 (got %d)", a->Cin);
@@ -1149,21 +1239,39 @@ extern "C" int av2v_gemm_f16(const av2v_gemm_args* a, av2v_stream_t stream_) {
   memset(&tr, 0, sizeof(tr));
   bool contig = true;
   if (a->mode == AV2V_A_CONV3X3) {  // p.W / p.H = output geometry
-    if (p.W > BM) contig = true;  // 128-pixel row segments in (frame, row, segment) order: output rows m_tile*128 ...
-    else if (p.frames_per_tile == 1) contig = (p.box_h * p.W == BM) && (p.H % p.box_h == 0);
-    else contig = (p.frames_per_tile * p.HW == BM);
+    // whole row segments / rows / frames that fill the tile and tile the image exactly: output rows m_tile*128 ... (3-D map)
+    if (p.frames_per_tile > 1) contig = (p.frames_per_tile * p.HW == BM);
+    else if (p.box_w * p.box_h != BM) contig = false;
+    else if (p.box_w == p.W) contig = (p.H % p.box_h == 0);
+    else contig = (p.box_h == 1 && p.W % p.box_w == 0);
+    p.block_store = (contig || p.up2) ? 0 : 1;
   } else if (a->mode == AV2V_A_TCONV3) {
     contig = (a->rows_per_clip % BM == 0);
   }
-  p.fast_epi = contig ? 1 : 0;
+  p.fast_epi = (contig || a->mode == AV2V_A_CONV3X3) ? 1 : 0;
+  p.o_box_bytes = p.block_store ? static_cast<uint32_t>(64 * p.box_w * p.box_h * p.frames_per_tile) : static_cast<uint32_t>(kEpiBufBytes);
   if (p.up2) {
-    // output = [NF][2H][2W][ldo]; the tile's rows (I = n*H + i, j) go to (2I + py, 2j + px): dims (c, px, j, py, I)
-    AV2V_REQUIRE(contig && p.W <= BM && BM % p.W == 0, AV2V_ENOSUP, "gemm/conv3x3 up2: needs tiles of whole image rows (W = %d)", p.W);
+    // output = [NF][2H][2W][N] (ldo == N); tile pixel (n, i, j) goes to (n, 2i + py, 2j + px): dims (px*N + c, j, py, i, n), so that
+    // the store box {32, box_w, 1, box_h, frames} is clipped at the right / bottom edge of the frame
     const uint64_t ld = static_cast<uint64_t>(a->ldo) * 2;
-    const uint64_t dims[5] = {static_cast<uint64_t>(a->N), 2, static_cast<uint64_t>(p.W), 2, static_cast<uint64_t>(p.NF) * p.H};
-    const uint64_t str[4] = {ld, 2 * ld, 2 * static_cast<uint64_t>(p.W) * ld, 4 * static_cast<uint64_t>(p.W) * ld};
-    const uint32_t box[5] = {32, 1, static_cast<uint32_t>(p.W), 1, static_cast<uint32_t>(BM / p.W)};
+    const uint64_t dims[5] = {2 * static_cast<uint64_t>(a->N), static_cast<uint64_t>(p.W), 2, static_cast<uint64_t>(p.H),
+                              static_cast<uint64_t>(p.NF)};
+    const uint64_t str[4] = {2 * ld, 2 * static_cast<uint64_t>(p.W) * ld, 4 * static_cast<uint64_t>(p.W) * ld,
+                             4 * static_cast<uint64_t>(p.HW) * ld};
+    const uint32_t box[5] = {32, static_cast<uint32_t>(p.box_w), 1, static_cast<uint32_t>(p.box_h), static_cast<uint32_t>(p.frames_per_tile)};
     if ((rc = make_tmap_f16(&to, a->out, 5, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B)) != AV2V_OK) return rc;
+  } else if (p.block_store) {
+    // [n_slots][NF][H][W][ldo] with box {32, box_w, box_h, frames, 1}: the out-of-image part of an edge block is not written
+    // (stores) or reads as zeros (residual loads)
+    const uint64_t ld = static_cast<uint64_t>(a->ldo) * 2;
+    const uint64_t slot_b = (a->n_slots > 1) ? static_cast<uint64_t>(a->slot_stride) * 2 : ld * static_cast<uint64_t>(a->M);
+    const uint64_t dims[5] = {static_cast<uint64_t>(a->N), static_cast<uint64_t>(p.W), static_cast<uint64_t>(p.H),
+                              static_cast<uint64_t>(p.NF), static_cast<uint64_t>(a->n_slots)};
+    const uint64_t str[4] = {ld, ld * p.W, ld * static_cast<uint64_t>(p.HW), slot_b};
+    const uint32_t box[5] = {32, static_cast<uint32_t>(p.box_w), static_cast<uint32_t>(p.box_h), static_cast<uint32_t>(p.frames_per_tile), 1};
+    if ((rc = make_tmap_f16(&to, a->out, 5, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B)) != AV2V_OK) return rc;
+    if (a->residual && (rc = make_tmap_f16(&tr, a->residual, 5, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B)) != AV2V_OK)
+      return rc;
   } else if (p.fast_epi) {
     const uint64_t slot_b = (a->n_slots > 1) ? static_cast<uint64_t>(a->slot_stride) * 2
                                              : static_cast<uint64_t>(a->ldo) * 2 * static_cast<uint64_t>(a->M);

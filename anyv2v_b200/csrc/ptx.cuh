@@ -365,7 +365,20 @@ __device__ __forceinline__ void tma_store_3d_w(uint32_t lead, const CUtensorMap*
       : "memory");
 }
 
-// 5-D tiled store (nearest-up x 2 fused into the conv: the tile's pixels go to every second pixel / row of the output image)
+// 5-D tiled load (the residual block of a conv tile: channels x columns x rows x frames x slot)
+__device__ __forceinline__ void tma_load_5d_w(uint32_t lead, uint32_t dst_addr, const CUtensorMap* m, uint32_t bar_addr, int c0,
+                                              int c1, int c2, int c3, int c4) {
+  asm volatile(
+      "{\n.reg .pred q;\n"
+      "setp.ne.b32 q, %8, 0;\n"
+      "@q cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];\n}\n" ::"r"(
+          dst_addr),
+      "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_addr), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4), "r"(lead)
+      : "memory");
+}
+
+// 5-D tiled store: a conv tile's block of pixels (channels x columns x rows x frames x slot), or with nearest-up x 2 fused into
+// the conv, every second pixel / row of the output image
 __device__ __forceinline__ void tma_store_5d_w(uint32_t lead, const CUtensorMap* m, uint32_t src_addr, int c0, int c1, int c2, int c3, int c4) {
   asm volatile(
       "{\n.reg .pred q;\n"

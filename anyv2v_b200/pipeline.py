@@ -186,6 +186,12 @@ class I2VGenXLPipeline:
             raise ValueError(f"`latents` must be [b, {self.unet.config['in_channels']}, f, h, w], got {tuple(latents.shape)}")
         if image_latents.shape[2:] != latents.shape[2:]:
             raise ValueError("`image_latents` and `latents` must agree in (frames, h, w)")
+        # every down block halves the latent and its up block doubles it back: odd sizes on the way down cannot be restored
+        f = 2 ** (len(self.unet.config["block_out_channels"]) - 1)
+        h, w = latents.shape[3], latents.shape[4]
+        if h % f or w % f:
+            raise ValueError(f"latent size {h} x {w} is not divisible by {f}: frame sides must be multiples of {8 * f} px "
+                             f"(64 px for I2VGen-XL, e.g. 1280 x 704), got {8 * w} x {8 * h} px")
 
     def _any_hook_fires(self, t) -> bool:
         mod = self.unet.up_blocks[1].resnets[1]

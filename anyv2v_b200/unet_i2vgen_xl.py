@@ -529,10 +529,7 @@ class Upsample2D(nn.Module):
         return self._phases.get(self.conv.weight, ops.pack_upsample_weights)
 
     def forward_nhwc(self, x):
-        nf, h, w, c = x.shape
-        if c % 64 == 0 and w <= 128 and 128 % w == 0 and ((h * w >= 128 and h % (128 // w) == 0) or (h * w < 128 and 128 % (h * w) == 0)):
-            return ops.upsample2x_conv3x3(x, self.phase_weights(), bias=self.conv.bias)
-        return self.conv.forward_nhwc(nr.nearest_up2_nhwc(x))  # geometries the fused tiles do not cover: materialise
+        return ops.upsample2x_conv3x3(x, self.phase_weights(), bias=self.conv.bias)
 
     def forward(self, x, output_size=None, scale: float = 1.0):
         return to_nchw_view(self.forward_nhwc(to_nhwc(x)))

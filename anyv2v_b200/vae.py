@@ -6,7 +6,8 @@ Module / parameter names are diffusers' (`encoder.down_blocks.0.resnets.0.norm1.
 `quant_conv`, `post_quant_conv`), so a real `diffusion_pytorch_model` state_dict loads unchanged.  Activations are
 channels-last fp16 end to end; every 3x3 convolution with Cin % 64 == 0 (all but `conv_in`), every GroupNorm(+SiLU),
 the 1x1 shortcuts and the attention projections run on `anyv2v_b200.ops` (tcgen05 implicit GEMM, fused bias/residual
-epilogue; image widths above 128 are tiled as 128-pixel row segments).  Left on library calls for now
+epilogue; a conv tile is a block of up to 128 pixels of one frame — 128-pixel row segments at widths that are multiples of
+128, 64 x 2 blocks at width 320, 32 x 4 at 160 — so any frame whose sides are multiples of 64 px runs).  Left on library calls for now
 (`next_rows`): `conv_in` (3 -> 128), the convolutions that end in 3 / 8 / 4 channels, the stride-2 down-sampling
 convolutions, and the single-head 512-wide mid-block attention core (head_dim 512 is outside the d = 64 kernel).
 There is no CPU path.

@@ -95,7 +95,7 @@ int av2v_groupnorm_silu_f16(const av2v_groupnorm_args* a, av2v_stream_t stream);
  *                                        + residual[slot][m, n]
  * A operand modes (all fed by TMA straight from the channels-last activation, no im2col buffer):
  *   AV2V_A_LINEAR : A is [M, K] row-major (lda elements)                      -> nn.Linear / 1x1 conv
- *   AV2V_A_CONV3X3: A is [NF, H, W, Cin]; K = 9*Cin, zero padding 1            -> Conv2d 3x3 (pnp_utils.py:78,107);
+ *   AV2V_A_CONV3X3: A is [NF, H, W, Cin]; K = 9*Cin, zero padding 1, any H, W -> Conv2d 3x3 (pnp_utils.py:78,107);
  *                   stride 2 (Downsample2D) samples the taps with TMA element strides; a_channels < Cin reads the
  *                   missing channels as zeros (conv_in: 8 channels in a 64-wide K block, weights zero-padded)
  *   AV2V_A_TCONV3 : A is [B, F*HW, Cin]; K = 3*Cin, zero padding over frames   -> Conv3d (3,1,1) of TemporalConvLayer
@@ -138,6 +138,17 @@ typedef struct {
                                      (2i+py, 2j+px) are written).  Four launches = the layer at 4/9 of its FLOPs. */
 } av2v_gemm_args;
 int av2v_gemm_f16(const av2v_gemm_args* a, av2v_stream_t stream);
+
+/* Tile plan of a CONV3X3 call, as av2v_gemm_f16 runs it.  One 128-row accumulator tile covers a block of box_h output rows x
+ * box_w output columns of one frame, or frames_per_tile (> 1) whole frames when a frame has at most 64 pixels.  Blocks at the
+ * right / bottom edge of a frame are partial (TMA clips their loads and stores).  Tiles are ordered (frame, row block,
+ * column block): tiles_per_frame = ceil(W_out / box_w) * ceil(H_out / box_h) (1 for whole frames), m_tiles tiles in all.
+ * av2v_conv3x3_plan validates the CONV3X3 fields of `a` exactly as av2v_gemm_f16 does (pointers are not looked at) and
+ * fills `out`; it makes no CUDA call. */
+typedef struct av2v_conv_plan {
+  int32_t box_w, box_h, frames_per_tile, tiles_per_frame, m_tiles;
+} av2v_conv_plan;
+int av2v_conv3x3_plan(const av2v_gemm_args* a, av2v_conv_plan* out);
 
 /* ------------------------------------------------------------------------------------------------------------
  * LayerNorm over the last dimension of a [rows, C] token matrix (norm1/norm2/norm3 of BasicTransformerBlock,

@@ -8,7 +8,9 @@ both epilogue groups of one CTA and checks them against the straightforward defi
   * the residual prefetch cursor — advanced independently, two loads ahead — produces exactly the (tile, chunk) sequence the group
     consumes, in the same buffer order;
   * with kOB output staging buffers, the store that last read a buffer was issued kOB chunks earlier by warp (turn - kOB) & 3, and that
-    warp's wait sits in the iteration before the buffer is staged again ((turn + 5 - kOB) & 3 == the issuer of chunk n - (kOB - 1)).
+    warp's wait sits in the iteration before the buffer is staged again ((turn + 5 - kOB) & 3 == the issuer of chunk n - (kOB - 1));
+  * block-shaped conv tiles (box_h x box_w pixels of one frame, or whole frames): the tile origin and per-row pixel the epilogue
+    derives cover every output pixel exactly once, and each tile's clipped store box holds exactly its valid rows.
 """
 from __future__ import annotations
 
@@ -108,6 +110,58 @@ def check(first_unit, stride, m_units, n_tiles, N, BN, geglu, k_ob=2):
     return sum(len(x) for x in sched)
 
 
+def conv_tile_origin(plan, W, m_tile):
+    """conv_tile_origin of the device code: first output pixel (n0, y0, x0) of a conv tile.  `plan` = (box_w, box_h,
+    frames_per_tile, tiles_per_frame, m_tiles) as av2v_conv3x3_plan returns it."""
+    box_w, box_h, fpt, tpf, _ = plan
+    if fpt > 1:
+        return m_tile * fpt, 0, 0
+    x_tiles = -(-W // box_w)
+    n0 = m_tile // tpf
+    yb, xb = divmod(m_tile - n0 * tpf, x_tiles)
+    return n0, yb * box_h, xb * box_w
+
+
+def block_tile_pixels(plan, NF, H, W, m_tile):
+    """the output pixels the epilogue writes for accumulator rows r = 0..127 of a block-shaped tile: {r: (n, y, x)} for the
+    rows it treats as valid (row-bias index, and the rows the clipped TMA store box keeps)"""
+    box_w, box_h, fpt, _, _ = plan
+    n0, y0, x0 = conv_tile_origin(plan, W, m_tile)
+    out = {}
+    for r in range(128):
+        bz, rr = divmod(r, box_w * box_h)
+        by, bx = divmod(rr, box_w)
+        n, y, x = n0 + bz, y0 + by, x0 + bx
+        if bz < fpt and x < W and y < H and n < NF:
+            out[r] = (n, y, x)
+    return out
+
+
+def check_block_tiles(plan, NF, H, W, pair=False):
+    """every output pixel is written by exactly one (tile, row); a tile's store box {box_w, box_h, frames} at its origin, clipped
+    to the image, holds exactly its valid rows (so a box never reaches into the next frame or row); rows are in the A box's
+    shared-memory order.  pair: the tile schedule of CTA pairs (2 mu + rank) including the phantom tile of an odd m_tiles."""
+    box_w, box_h, fpt, tpf, m_tiles = plan
+    assert box_w * box_h * fpt <= 128 and max(box_w, box_h, fpt) <= 256
+    seen = {}
+    tiles = range(2 * (-(-m_tiles // 2))) if pair else range(m_tiles)
+    for m in tiles:
+        px = block_tile_pixels(plan, NF, H, W, m)
+        if m >= m_tiles:
+            assert not px, f"phantom pair tile {m} writes {len(px)} pixels"
+            continue
+        n0, y0, x0 = conv_tile_origin(plan, W, m)
+        assert n0 < NF and y0 < H and x0 < W, (m, n0, y0, x0)
+        box = {(n, y, x) for n in range(n0, min(n0 + fpt, NF)) for y in range(y0, min(y0 + box_h, H))
+               for x in range(x0, min(x0 + box_w, W))}
+        assert set(px.values()) == box, (m, len(px), len(box))
+        for r, pix in px.items():
+            assert pix not in seen, f"pixel {pix} written by tiles {seen[pix]} and {m}"
+            seen[pix] = m
+    assert len(seen) == NF * H * W, (len(seen), NF * H * W)
+    return len(seen)
+
+
 if __name__ == "__main__":
     total = 0
     for BN, N, geglu in ((160, 960, False), (160, 320, False), (256, 2560, True), (128, 320, False), (64, 200, False), (256, 1280, False), (128, 1280, True)):
@@ -116,3 +170,7 @@ if __name__ == "__main__":
             for k_ob in (2, 3):
                 total += check(first, stride, m_units, n_tiles, N, BN, geglu, k_ob)
     print(f"lean epilogue bookkeeping: {total} chunk visits checked")
+    # block tiles of 1280 x 704 (latent 160 x 88 and its levels): plans as av2v_conv3x3_plan returns them
+    px = sum(check_block_tiles(plan, 3, H, W, pair=True) for plan, H, W in (((32, 4, 1, 110, 330), 88, 160), ((16, 8, 1, 30, 90), 44, 80),
+                                                                             ((40, 3, 1, 8, 24), 22, 40), ((20, 6, 1, 2, 6), 11, 20)))
+    print(f"block conv tiles: {px} output pixels covered exactly once")

@@ -111,6 +111,98 @@ def census(batch, inject):
     return calls
 
 
+def _conv_stubs(convs):
+    """shape-only stand-ins for every anyv2v_b200.ops entry the UNet / VAE forward passes call; the 3x3 convolutions (plain,
+    strided and the four phases of the fused Upsample2D) are recorded as av2v_gemm_args field dicts"""
+    empty = lambda shape, like: torch.empty(shape, dtype=torch.float16, device=like.device)
+
+    def linear(a, w, bias=None, residual=None, out=None, rowbias=None, rows_per_rowbias=0, geglu=False, a2=None):
+        return out if out is not None else empty((a.shape[0], w.shape[0] // 2 if geglu else w.shape[0]), a)
+
+    def conv3x3(x, w, bias=None, rowbias=None, rows_per_rowbias=0, residual=None, out=None, n_slots=1, slot_stride=0, stride=1):
+        NF, H, W, C = x.shape
+        Cout, Cin = w.shape[0], w.shape[1] // 9
+        convs.append(dict(NF=NF, H=H, W=W, Cin=Cin, N=Cout, K=9 * Cin, M=NF * (H // stride) * (W // stride), stride=stride,
+                          a_channels=C if C != Cin else 0, ldo=Cout, n_slots=n_slots, residual=residual is not None,
+                          rowbias=rowbias is not None, up2_phase=0))
+        return out if out is not None else empty((NF, H // stride, W // stride, Cout), x)
+
+    def upsample2x_conv3x3(x, w_phases, bias=None, out=None):
+        NF, H, W, Cin = x.shape
+        Cout = w_phases.shape[1]
+        for ph in range(4):
+            convs.append(dict(NF=NF, H=H, W=W, Cin=Cin, N=Cout, K=4 * Cin, M=NF * H * W, stride=1, a_channels=0, ldo=Cout, n_slots=1,
+                              residual=False, rowbias=False, up2_phase=ph + 1))
+        return out if out is not None else empty((NF, 2 * H, 2 * W, Cout), x)
+
+    def tconv3(x, w, F, HW, bias=None, residual=None, out=None):
+        return out if out is not None else empty((x.shape[0], x.shape[1], w.shape[0]), x)
+
+    def groupnorm(x, g, b, groups, eps, silu, out=None, x2=None):
+        return empty(x.shape[:-1] + (x.shape[-1] + (x2.shape[-1] if x2 is not None else 0),), x)
+
+    def layernorm(x, g, b, eps=1e-5, out=None):
+        return torch.empty_like(x)
+
+    def attention(q, k, v, heads, seq, batch, out, **kw):
+        return out
+
+    def temporal_attention_fused(x, wqkv, heads, F, HW, clips, out, **kw):
+        return out
+
+    return dict(linear=linear, conv3x3=conv3x3, upsample2x_conv3x3=upsample2x_conv3x3, tconv3=tconv3, groupnorm=groupnorm,
+                layernorm=layernorm, attention=attention, temporal_attention_fused=temporal_attention_fused)
+
+
+def _with_stubs(convs, fn):
+    from anyv2v_b200 import ops
+    stubs = _conv_stubs(convs)
+    saved = {n: getattr(ops, n) for n in stubs}
+    for n, f in stubs.items():
+        setattr(ops, n, f)
+    try:
+        with torch.no_grad():
+            fn()
+    finally:
+        for n, f in saved.items():
+            setattr(ops, n, f)
+    return convs
+
+
+def unet_conv_census(batch, inject, frames, height, width):
+    """every 3x3 convolution of one full-size UNet forward at latent height x width: an inversion step (batch 1) or a PnP edit
+    step (batch 3, conv + spatial injection firing)"""
+    from anyv2v_b200 import pnp_utils
+    from anyv2v_b200.unet_i2vgen_xl import I2VGEN_XL_CONFIG, I2VGenXLUNet
+
+    def run():
+        with torch.device("meta"):
+            net = I2VGenXLUNet(**I2VGEN_XL_CONFIG).half()
+        m = lambda *s: torch.empty(*s, dtype=torch.float16, device="meta")
+        if inject:
+            pipe = SimpleNamespace(unet=net)
+            pnp_utils.register_conv_injection(pipe, [981])
+            pnp_utils.register_spatial_attention_pnp(pipe, [981])
+            pnp_utils.register_temp_attention_pnp(pipe, [981])
+            pnp_utils.register_time(pipe, 981)
+        cond = dict(fps_emb=m(batch, 1280), ctx=m(batch, 145, 1024), image_latents_nhwc=m(batch * frames, height, width, 4))
+        net(m(batch, 4, frames, height, width), torch.empty(1, dtype=torch.int64, device="meta"), cond=cond)
+    return _with_stubs([], run)
+
+
+def vae_conv_census(frames, height, width):
+    """every 3x3 convolution the VAE runs on the tensor cores for an encode of `frames` height x width frames and the decode
+    of their latents"""
+    from anyv2v_b200.vae import SD_VAE_CONFIG, AutoencoderKL
+
+    def run():
+        with torch.device("meta"):
+            vae = AutoencoderKL(**SD_VAE_CONFIG).half()
+        vae.encode(torch.empty(frames, 3, height, width, dtype=torch.float16, device="meta"))
+        vae.decode(torch.empty(frames, 4, height // 8, width // 8, dtype=torch.float16, device="meta"))
+    return _with_stubs([], run)
+
+
 def report(title, calls):
     gemms = OrderedDict()
     for name, mode, M, N, K, m_tiles, geglu in calls:
